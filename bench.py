@@ -365,6 +365,23 @@ def roofline_from(rep, B, L_by_stack, precision, peaks, peaks_src, tot_ms):
                                                                   "tflops": round(c["flops"] / (c["ms_pair"] * 1e-3) / 1e12, 1)} for c in cands}}}
 
 
+DUMP_LIMIT = 64 * 10 ** 6           # bytes --dump-outputs writes at most
+
+
+def dump_outputs(out_dir, waveforms):
+    """--dump-outputs: the (utterances, samples) float32 waveforms a caller of the timed path receives, from its last
+    step, as waveforms.npy.  Above DUMP_LIMIT: a fixed seeded sample of the flattened array, with the flat indices it
+    took (ascending) in waveforms_index.npy."""
+    os.makedirs(out_dir, exist_ok=True)
+    y = waveforms.float().cpu().numpy()
+    if y.nbytes > DUMP_LIMIT:
+        n = (DUMP_LIMIT - 4096) // (y.itemsize + 8)                     # 4096: room for the two .npy headers
+        idx = np.sort(np.random.default_rng(0).choice(y.size, n, replace=False))
+        np.save(os.path.join(out_dir, "waveforms_index.npy"), idx.astype(np.float64))
+        y = y.reshape(-1)[idx]
+    np.save(os.path.join(out_dir, "waveforms.npy"), y)
+
+
 def measure_batch(args, precision, rank, world, local, B, full=True):
     """One engine at `precision`: resident and end-to-end throughput of the batch step (see the module docstring)."""
     import torch.distributed as dist
@@ -424,6 +441,7 @@ def measure_batch(args, precision, rank, world, local, B, full=True):
         ev_ready = torch.cuda.Event()
         host_full = torch.empty(world * B, L).pin_memory() if rank == 0 else None
     counter = [0]
+    gathered = [None]
 
     def step(e2e):
         k = counter[0] & 1
@@ -442,7 +460,7 @@ def measure_batch(args, precision, rank, world, local, B, full=True):
         ev_ready.record(main)
         with torch.cuda.stream(comm):
             comm.wait_event(ev_ready)
-            y = gplan(gsrc[k])
+            y = gathered[0] = gplan(gsrc[k])
             if e2e and rank == 0:
                 host_full.copy_(y, non_blocking=True)                   # rank 0 reads back the WHOLE gathered result
             ev_done[k].record(comm)
@@ -469,6 +487,8 @@ def measure_batch(args, precision, rank, world, local, B, full=True):
         sampler.start()
     ms_step = timed(False, args.steps) / args.steps
     clocks = sampler.stop() if rank == 0 and full else None
+    if rank == 0 and full and args.dump_outputs:
+        dump_outputs(args.dump_outputs, dev_out if world == 1 else gathered[0])
     l0 = eng.launch_count(); eng.restore(dev_in, mode=0, out=dev_out); torch.cuda.synchronize()
     launches = (eng.launch_count() - l0) * args.steps                  # graph replays bypass the library's counter
     audio_per_step = world * B * args.seconds
@@ -571,7 +591,12 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the second precision mode, the workloads and the library baseline")
     ap.add_argument("--no-graph", action="store_true", help="launch the kernels of a step individually")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the waveforms of the last timed step to DIR/waveforms.npy (float32; over 64 MB, a fixed "
+                         "seeded sample), to compare two builds output for output")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs applies to --impl b200")
     if args.impl == "reference":
         if not args.batch:
             args.batch = 32 if args.gpus == 1 else 64

@@ -3,20 +3,18 @@
 The reference's acceptance test is FLAC in / FLAC out through librosa.load and soundfile.write
 (test/test.py:48-57,85-89; voicefixer/base.py:47-49; tools/wav.py:37).  The decoder is pinned by
 (a) a libFLAC-encoded excerpt of the reference's own test input with the PCM of its sibling .wav
-(tests/golden/flac_libflac_excerpt.npz, made by tests/golden/make_flac_golden.py), (b) when
-/root/reference is present, every .flac the reference ships, against the MD5 signature libFLAC
-stored in STREAMINFO, and (c) hashlib for the MD5 itself.  The encoder is pinned by the decoder."""
-import glob
+(tests/golden/flac_libflac_excerpt.npz, made by tests/golden/make_flac_golden.py), (b) frames of
+every .flac the reference ships, against the header and MD5 signatures libFLAC stored in STREAMINFO
+(tests/golden/flac_reference_excerpts.npz, same script), and (c) hashlib for the MD5 itself.  The
+encoder is pinned by the decoder."""
 import hashlib
 import os
 import re
-import wave
 
 import numpy as np
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF_UTT = "/root/reference/test/utterance"
 
 
 def test_hostio_library_exports_every_declared_symbol():
@@ -140,26 +138,32 @@ def test_wavio_flac_follows_the_file_extension(tmp_path):
     assert m.shape == (60000,)
 
 
-@pytest.mark.skipif(not os.path.isdir(REF_UTT), reason="reference checkout not present (GPU box)")
-def test_decode_every_reference_flac_against_its_libflac_md5():
-    """All FLAC files the reference ships (inputs, targets, outputs): header fields, frame CRCs and the MD5
-    signature written by libFLAC; sample counts are the ones BASELINE.md quotes; original.flac == original.wav."""
+def test_decode_every_reference_flac_against_its_libflac_md5(tmp_path):
+    """Every distinct FLAC file the reference ships (inputs, targets, outputs), as tests/golden/make_flac_golden.py
+    stored it: the metadata chain libFLAC wrote (header fields, the sample counts BASELINE.md quotes, an MD5
+    signature), and the file's first, middle and last frames with frame CRCs and the MD5 of those frames' audio,
+    taken from a full decode that matched libFLAC's signature; original.flac's frames == original.wav's samples."""
     from voicefixer_b200 import _hostio, wavio
-    files = sorted(glob.glob(os.path.join(REF_UTT, "*", "*.flac")))
+    g = np.load(os.path.join(ROOT, "tests", "golden", "flac_reference_excerpts.npz"))
+    files = [str(f) for f in g["files"]]
     assert len(files) >= 6
     expect = {"original.flac": 132300, "p360_001_mic1.flac": 96076, "oracle.flac": 97902, "output_mode_0.flac": 132300,
               "output_mode_1.flac": 132096, "output_mode_2.flac": 132300}
-    for f in files:
-        data = open(f, "rb").read()
-        info = _hostio.flac_info(data)
+    for i, f in enumerate(files):
+        info = _hostio.flac_info(g[f"header{i}"].tobytes())
+        n, bs = expect[os.path.basename(f)], info.max_blocksize
+        assert (info.sample_rate, info.channels, info.bits_per_sample, info.total_samples) == (44100, 1, 16, n), f
         assert any(info.md5), f
+        data = g[f"excerpt{i}"].tobytes()
         pcm, sr, bps = _hostio.flac_decode(data)                     # raises on CRC / MD5 mismatch
-        assert (sr, bps, pcm.shape) == (44100, 16, (expect[os.path.basename(f)], 1)), f
-        assert hashlib.md5(pcm.astype("<i2").tobytes()).digest() == bytes(info.md5)
-    with wave.open(os.path.join(REF_UTT, "original", "original.wav"), "rb") as w:
-        ref = np.frombuffer(w.readframes(w.getnframes()), dtype="<i2")
-    got = wavio.load_mono(os.path.join(REF_UTT, "original", "original.flac"))
-    assert np.array_equal(got, ref.astype(np.float32) / 32768.0)
+        want = sum(min(bs, n - k * bs) for k in g[f"frames{i}"])
+        assert g[f"frames{i}"][-1] == (n - 1) // bs                  # the ragged last block is among them
+        assert (sr, bps, pcm.shape) == (44100, 16, (want, 1)), f
+        assert hashlib.md5(pcm.astype("<i2").tobytes()).digest() == bytes(_hostio.flac_info(data).md5)
+        if os.path.basename(f) == "original.flac":
+            (tmp_path / "original.flac").write_bytes(data)
+            got = wavio.load_mono(str(tmp_path / "original.flac"))
+            assert np.array_equal(got, g["original_wav"].astype(np.float32) / 32768.0)
 
 
 # ------------------------------------------------------------------ decoder paths no available file reaches

@@ -1,12 +1,13 @@
 """CPU tests: the oracle restatement against the golden vectors produced by the UNMODIFIED
 reference (tests/golden/make_golden.py), plus the length arithmetic pinned by the reference's
 own FLAC fixtures (SURVEY 8c)."""
+import importlib.util
 import os
 
 import numpy as np
 import torch
 import pytest
-from conftest import golden, rel_rms
+from conftest import GOLDEN, golden, rel_rms
 from oracle import vf_oracle as O
 
 
@@ -103,25 +104,20 @@ def test_slaney_basis_matches_torchaudio_formula():
     assert np.max(np.abs(O.slaney_htk_mel_basis() - ref)) < 2e-6
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/voicefixer"), reason="reference checkout not present (GPU box)")
+def _live_pin():
+    """tests/golden/live_pin.py: regenerates the inputs of live_pin.npz and runs the oracle on them."""
+    spec = importlib.util.spec_from_file_location("live_pin", os.path.join(GOLDEN, "live_pin.py"))
+    mod = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(mod)
+    return mod
+
+
 def test_slaney_basis_matches_the_reference_melscale_fbanks():
     """The one independent cross-check of Vocoder.oracle()'s mel basis that exists offline (librosa is absent): the
     reference's OWN implementation of the same filterbank, melscale_fbanks(..., norm="slaney", mel_scale="htk")
-    (voicefixer/tools/mel_scale.py:173-238, Slaney branch :226-229), imported unmodified from /root/reference and
-    run here -- against both the oracle's and the product's (wavio) restatement of librosa.filters.mel."""
-    import subprocess, sys, json
-    code = (
-        "import sys, json, numpy as np; sys.path.insert(0, %r)\n"
-        "from ref_loader import install; install()\n"
-        "from voicefixer.tools.mel_scale import melscale_fbanks\n"
-        "fb = melscale_fbanks(1025, 0.0, 22050.0, 128, 44100, norm='slaney', mel_scale='htk')\n"
-        "np.save(sys.argv[1], fb.numpy())\n") % os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
-    import tempfile
-    with tempfile.TemporaryDirectory() as td:
-        out = os.path.join(td, "fb.npy")
-        r = subprocess.run([sys.executable, "-c", code, out], capture_output=True, text=True, timeout=120)
-        assert r.returncode == 0, r.stderr[-2000:]
-        ref = np.load(out).T                                        # (128, 1025) like librosa.filters.mel
+    (voicefixer/tools/mel_scale.py:173-238, Slaney branch :226-229), run unmodified by tests/golden/live_pin.py and
+    stored in live_pin.npz -- against both the oracle's and the product's (wavio) restatement of librosa.filters.mel."""
+    ref = _live_pin().stored_filterbank(golden("live_pin")).T      # (128, 1025) like librosa.filters.mel
     from voicefixer_b200 import wavio
     assert ref.shape == (128, 1025)
     scale = float(np.max(np.abs(ref)))
@@ -131,18 +127,19 @@ def test_slaney_basis_matches_the_reference_melscale_fbanks():
 
 
 @pytest.mark.timeout(900)
-@pytest.mark.skipif(not os.path.isdir("/root/reference/voicefixer"), reason="reference checkout not present (GPU box)")
-def test_oracle_live_against_unmodified_reference_on_fresh_inputs():
-    """tests/golden/live_pin.py: the unmodified reference (its own VoiceFixer() / Vocoder() loading seeded synthetic
-    checkpoints) against the oracle on inputs that are not in the committed fixtures -- analysis at the 64-frame grid
-    edges, vocoder at odd / even T, restore_inmem modes 0 and 2 (with the dropout masks the reference drew), and the
-    your_vocoder_func hook.  Run in a subprocess: the stub-loader registers a `voicefixer` namespace package."""
-    import json, subprocess, sys
-    script = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "live_pin.py")
-    r = subprocess.run([sys.executable, script, "9100"], capture_output=True, text=True, timeout=850)
-    assert r.returncode == 0, r.stderr[-3000:]
-    rep = json.loads(r.stdout.strip().splitlines()[-1])
-    assert set(rep) >= {"analysis_T2", "analysis_T64", "analysis_T128", "analysis_T257", "vocoder_T5", "vocoder_T12",
+def test_oracle_live_against_unmodified_reference_on_fresh_inputs(states):
+    """The oracle against what the unmodified reference (its own VoiceFixer() / Vocoder() loading seeded synthetic
+    checkpoints) computed on inputs that are not in the other fixtures -- analysis at the 64-frame grid edges, vocoder
+    at odd / even T, restore_inmem modes 0 and 2 (with the dropout masks the reference drew), and the your_vocoder_func
+    hook.  tests/golden/live_pin.py ran the reference and stored a fixed sample of every output in live_pin.npz."""
+    lp, g = _live_pin(), golden("live_pin")
+    x = lp.inputs(int(g["seed"]))
+    for k, v in x.items():                                              # the inputs the reference saw
+        assert np.isclose(np.sum(np.asarray(v, np.float64)), g["insum_" + k], rtol=1e-12, atol=0), k
+    out = lp.oracle_outputs(x, states[0], states[1], lp.stored_masks(g))
+    assert set(out) == {"analysis_T2", "analysis_T64", "analysis_T128", "analysis_T257", "vocoder_T5", "vocoder_T12",
                         "restore_mode0_1.3s", "restore_mode2_1.6s", "hook_mel", "hook_out"}
-    for k, v in rep.items():
-        assert v < (2e-5 if k != "hook_mel" else 5e-5), (k, v)             # fp32 restatement: same ops, same order
+    for k, v in out.items():
+        assert v.shape == tuple(g["shape_" + k]), k
+        err = rel_rms(lp.sample(v), g["ref_" + k])
+        assert err < (2e-5 if k != "hook_mel" else 5e-5), (k, err)     # fp32 restatement: same ops, same order
